@@ -2,6 +2,7 @@
 """bench.py -- the protein-to-genome mapping hot path on N B200s (BASELINE.json metric: proteins/s, DP Gcell/s).
 
   python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--workload C2|C5|C4s|C3s|small|tiny]
+                  [--dump-outputs DIR]
 
 One "step" = one pass of the hot path (seed + chain + refine + nasw DP waves + host bookkeeping) over one batch of
 synthetic proteins of the named workload (C2 = BASELINE.json configs[1]: 100 Mbp genome, 1000 proteins of ~400 aa per GPU).
@@ -18,7 +19,12 @@ proteins: the N shards of 1000 proteins each.
              with its index loaded once before the timed region.
 
 What a process pays once (context creation, index load, upload / broadcast) is reported separately under `process`.
-The PAF of EVERY rank is compared with the reference's output for that rank's shard; a mismatch fails the run.
+The PAF of EVERY rank is compared with the reference's output for that rank's shard, where the reference is built; a mismatch
+fails the run.
+
+--dump-outputs DIR writes what the last timed `value` step returned to its caller (rank 0's regions: coordinates, scores,
+alignment statistics, CIGARs, exon features) as DIR/<name>.npy in float64, so that two builds can be compared output for output
+on the same seeded inputs.
 """
 from __future__ import annotations
 
@@ -93,6 +99,72 @@ def prepare(workload, rank, world):
         for r in range(world):
             synth.shard_queries(spec, d, r)
     return spec, d
+
+
+class Extra(C.Structure):  # mp_extra_t (include/miniprot_b200.h), followed by n_cigar uint32 CIGAR words
+    _fields_ = [(f, C.c_int32) for f in ("dp_score", "dp_max", "dp_max2", "n_cigar", "m_cigar", "blen", "n_fs", "n_stop", "dist_stop",
+                                         "dist_start", "n_iden", "n_plus")]
+
+
+class Feat(C.Structure):  # mp_feat_t
+    _fields_ = [("vs", C.c_int64), ("ve", C.c_int64), ("qs", C.c_int32), ("qe", C.c_int32), ("type", C.c_int16), ("phase", C.c_int16),
+                ("n_fs", C.c_int32), ("n_stop", C.c_int32), ("score", C.c_int32), ("n_iden", C.c_int32), ("blen", C.c_int32),
+                ("donor", C.c_char * 2), ("acceptor", C.c_char * 2)]
+
+
+class Reg1(C.Structure):  # mp_reg1_t
+    _fields_ = [(f, C.c_int32) for f in ("off", "cnt", "id", "parent", "n_sub", "subsc", "n_feat", "m_feat", "n_exon", "chn_sc", "chn_sc_ungap")] + \
+        [("hash", C.c_uint32), ("vid", C.c_uint32), ("qs", C.c_int32), ("qe", C.c_int32), ("vs", C.c_int64), ("ve", C.c_int64),
+         ("a", C.c_void_p), ("feat", C.POINTER(Feat)), ("p", C.POINTER(Extra))]
+
+
+REG_FIELDS = ("vid", "qs", "qe", "vs", "ve", "id", "parent", "n_sub", "subsc", "cnt", "n_exon", "n_feat", "chn_sc", "chn_sc_ungap", "hash")
+EXTRA_FIELDS = ("dp_score", "dp_max", "dp_max2", "n_cigar", "blen", "n_fs", "n_stop", "dist_stop", "dist_start", "n_iden", "n_plus")
+FEAT_FIELDS = ("vs", "ve", "qs", "qe", "type", "phase", "n_fs", "n_stop", "score", "n_iden", "blen")
+DUMP_LIMIT = 64 << 20
+
+
+def dump_regions(out_dir, n, n_reg, regs):
+    """Every region of every protein (reg_*: one row per region, protein by protein; reg_qid = the protein's index in the batch,
+    reg_has_extra = 0 where the region carries no alignment), the alignment statistics (ext_*), the CIGAR words of all regions
+    concatenated (cigar, with reg_cigar_off), and the exon features (feat_*, with reg_feat_off).  All float64 (exact for these
+    integers).  Above 64 MB in all, a fixed seeded sample of the proteins is written instead."""
+    import numpy as np
+
+    def arrays(qids):
+        cols = {k: [] for k in ("reg_qid", "reg_has_extra", "reg_cigar_off", "reg_feat_off", "cigar")}
+        cols.update({"reg_" + f: [] for f in REG_FIELDS})
+        cols.update({"ext_" + f: [] for f in EXTRA_FIELDS})
+        cols.update({"feat_" + f: [] for f in FEAT_FIELDS})
+        for i in qids:
+            rs = C.cast(regs[i], C.POINTER(Reg1))
+            for j in range(n_reg[i]):
+                r = rs[j]
+                cols["reg_qid"].append(i)
+                for f in REG_FIELDS:
+                    cols["reg_" + f].append(getattr(r, f))
+                cols["reg_cigar_off"].append(len(cols["cigar"]))
+                cols["reg_feat_off"].append(len(cols["feat_vs"]))
+                cols["reg_has_extra"].append(1 if r.p else 0)
+                e = r.p.contents if r.p else Extra()
+                for f in EXTRA_FIELDS:
+                    cols["ext_" + f].append(getattr(e, f))
+                if r.p and e.n_cigar:
+                    cig = C.cast(C.addressof(e) + C.sizeof(Extra), C.POINTER(C.c_uint32 * e.n_cigar)).contents
+                    cols["cigar"].extend(cig)
+                for k in range(r.n_feat if r.feat else 0):
+                    for f in FEAT_FIELDS:
+                        cols["feat_" + f].append(getattr(r.feat[k], f))
+        return {k: np.asarray(v, dtype=np.float64) for k, v in cols.items()}
+
+    out = arrays(range(n))
+    total = sum(a.nbytes for a in out.values())
+    if total > DUMP_LIMIT:
+        keep = np.sort(np.random.default_rng(0).permutation(n)[:max(1, int(n * DUMP_LIMIT / total * 0.9))])
+        out = arrays(keep)
+    os.makedirs(out_dir, exist_ok=True)
+    for k, a in out.items():
+        np.save(os.path.join(out_dir, k + ".npy"), a)
 
 
 def workload_text(name, spec, n_per_gpu, world):
@@ -214,7 +286,10 @@ def main():
     ap.add_argument("--warmup", type=int, default=3)
     ap.add_argument("--impl", default="ours", choices=["ours", "reference"])
     ap.add_argument("--workload", default="C2")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None, help="write rank 0's results of the last timed step as DIR/<name>.npy")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
     rank, world = int(os.environ.get("RANK", 0)), int(os.environ.get("WORLD_SIZE", 1))
     local = int(os.environ.get("LOCAL_RANK", 0))
 
@@ -315,11 +390,13 @@ def main():
     regs = (C.c_void_p * n)()
     out_paf = os.path.join(d, f"ours.rank{rank}.paf")
 
-    def step_resident():
+    def step_resident(keep=False):
+        """keep: leave the regions to the caller (the last timed step: dumped if asked, and freed, after the timed region)."""
         assert L.mpb_map_batch(ctx.h, mi, C.byref(mo), n, c_seqs, c_lens, c_names, n_reg, regs) == 0
-        L.mpb_regs_free(n, n_reg, regs)
+        if not keep:
+            L.mpb_regs_free(n, n_reg, regs)
 
-    def step_e2e():
+    def step_e2e(keep=False):
         mp.map_file(ctx, mi, prot, out_paf, mo)
 
     def timed(fn, steps):
@@ -330,8 +407,8 @@ def main():
         torch.cuda.synchronize()
         L.mpb_event_begin(ctx.h)
         t0 = time.perf_counter()
-        for _ in range(steps):
-            fn()
+        for i in range(steps):
+            fn(keep=i == steps - 1)
         ms = L.mpb_event_end_ms(ctx.h)
         torch.cuda.synchronize()
         wall = (time.perf_counter() - t0) * 1e3
@@ -354,6 +431,9 @@ def main():
         sampler.start()
     ms, ms_mine = timed(step_resident, args.steps)
     st = ctx.stats()
+    if args.dump_outputs is not None and rank == 0:
+        dump_regions(args.dump_outputs, n, n_reg, regs)
+    L.mpb_regs_free(n, n_reg, regs)
     step_e2e()
     ctx.reset_stats()
     ms_e2e, ms_e2e_mine = timed(step_e2e, args.steps)

@@ -4,12 +4,22 @@
 * ``oracle/liboracle.so``    - the plain-C restatement of the hot path
 
 plus seeded random problem generators shared by the CPU and GPU parity tests.
+
+Every answer of the reference goes through ``reference()``: where oracle/_ref is built the reference is called, elsewhere the
+answer it gave on the same inputs is read from tests/golden/reference_results.json.gz.  Record that file (merged with what it
+holds) by running the tests where oracle/_ref is built with MPB_RECORD_REFERENCE=1.
 """
 from __future__ import annotations
 
+import atexit
+import base64
 import ctypes as C
+import gzip
+import hashlib
+import json
 import os
 import subprocess
+import time
 
 import numpy as np
 
@@ -18,6 +28,100 @@ ORA_DIR = os.path.join(ROOT, "oracle")
 REF_SO = os.path.join(ORA_DIR, "_ref", "libref.so")
 REF_BIN = os.path.join(ORA_DIR, "_ref", "miniprot")
 ORA_SO = os.path.join(ORA_DIR, "liboracle.so")
+GOLDEN = os.path.join(ROOT, "tests", "golden")
+RECORDED = os.path.join(GOLDEN, "reference_results.json.gz")
+# the reference's two bundled test inputs (data)
+DPP3_GEN, DPP3_PEP = os.path.join(GOLDEN, "DPP3-hs.gen.fa.gz"), os.path.join(GOLDEN, "DPP3-mm.pep.fa.gz")
+
+_recorded = None
+_record = os.environ.get("MPB_RECORD_REFERENCE") == "1"
+
+
+def _save_recorded():
+    with open(RECORDED, "wb") as f, gzip.GzipFile(fileobj=f, mode="wb", mtime=0) as z:
+        z.write(json.dumps(_recorded, sort_keys=True, separators=(",", ":")).encode())
+
+
+def _canon(x):
+    """x as plain JSON data (numpy scalars as Python numbers, byte strings and ctypes arrays as their sha256, ctypes structures
+    as field dicts), so that a key does not depend on how a value prints."""
+    if isinstance(x, (bytes, bytearray, memoryview)):
+        return "sha256:" + digest(x)
+    if isinstance(x, (bool, np.bool_)):
+        return bool(x)
+    if isinstance(x, (int, np.integer)):
+        return int(x)
+    if isinstance(x, (float, np.floating)):
+        return float(x)
+    if isinstance(x, C.Structure):
+        return {f: _canon(getattr(x, f)) for f, _ in x._fields_}
+    if isinstance(x, C.Array):
+        return _canon(bytes(x))
+    if isinstance(x, dict):
+        return {str(k): _canon(v) for k, v in x.items()}
+    if isinstance(x, (list, tuple)):
+        return [_canon(v) for v in x]
+    if x is None or isinstance(x, str):
+        return x
+    raise TypeError(f"no canonical form for {type(x).__name__}")
+
+
+def reference(kind: str, parts, compute):
+    """The reference's answer (JSON data) to one call identified by `kind` and its inputs `parts`: compute() where the reference
+    is built -- checked against the answer recorded for the same inputs, if there is one -- else the recorded answer."""
+    global _recorded
+    key = f"{kind}:" + hashlib.sha256(json.dumps([kind, _canon(list(parts))], sort_keys=True).encode()).hexdigest()[:32]
+    if _recorded is None:
+        _recorded = json.loads(gzip.open(RECORDED).read()) if os.path.exists(RECORDED) else {}
+        if _record:
+            atexit.register(_save_recorded)
+    if have_ref():
+        v = json.loads(json.dumps(compute()))  # the same types as a recorded answer
+        if _record:
+            _recorded[key] = v
+        elif key in _recorded and _recorded[key] != v:
+            raise AssertionError(f"the reference now answers this {kind} call ({key}) differently from the answer recorded in "
+                                 f"{os.path.relpath(RECORDED, ROOT)}: record it again (MPB_RECORD_REFERENCE=1)")
+        return v
+    if key not in _recorded:
+        raise KeyError(f"no recorded answer of the reference for this {kind} call ({key}): record it where oracle/_ref is built "
+                       f"(MPB_RECORD_REFERENCE=1)")
+    return _recorded[key]
+
+
+def digest(b) -> str:
+    return hashlib.sha256(bytes(b)).hexdigest()
+
+
+def file_digest(path: str) -> str:
+    h = hashlib.sha256()
+    with open(path, "rb") as f:
+        for blk in iter(lambda: f.read(1 << 24), b""):
+            h.update(blk)
+    return h.hexdigest()
+
+
+def ref_cli(args, g, p, threads=8, index=None) -> dict:
+    """md5 and line count of what the reference CLI prints for `args` on genome `g` and proteins `p`; where the reference is run
+    here also `out`, `err` and `s`: its stdout, its stderr and its wall time in seconds.  index: an .mpi of `g` for the reference to restore instead of indexing g
+    (the index file is part of the reference's contract: tests/test_tables.py::test_index_file_is_byte_identical)."""
+    out = {}
+
+    def run():
+        t0 = time.perf_counter()
+        r = subprocess.run([REF_BIN, f"-t{threads}", *args, index or g, p], check=True, capture_output=True)
+        out["out"], out["err"], out["s"] = r.stdout, r.stderr, time.perf_counter() - t0
+        return {"md5": hashlib.md5(r.stdout).hexdigest(), "lines": r.stdout.count(b"\n")}
+
+    return dict(reference("cli", (list(args), file_digest(g), file_digest(p)), run), **out)
+
+
+def _b64(a: np.ndarray) -> str:
+    return base64.b64encode(np.ascontiguousarray(a).tobytes()).decode()
+
+
+def _unb64(s: str, dtype) -> np.ndarray:
+    return np.frombuffer(base64.b64decode(s), dtype=dtype).copy()
 
 
 def build_oracle():
@@ -99,14 +203,19 @@ def ora():
     return _ora
 
 
+_TAB_SIZES = (("nt4", 256), ("aa20", 256), ("aa13", 256), ("codon", 64), ("codon13", 64))
+_ref_tab = None
+
+
 def ref_tables() -> OraTab:
-    """Oracle table bundle pointing at the REFERENCE's tables (after ref_mp_start())."""
-    r = ref()
-    t = OraTab()
-    for f, sym in (("nt4", "ref_ns_tab_nt4"), ("aa20", "ref_ns_tab_aa20"), ("aa13", "ref_ns_tab_aa13"),
-                   ("codon", "ref_ns_tab_codon"), ("codon13", "ref_ns_tab_codon13")):
-        setattr(t, f, C.addressof(C.c_uint8.in_dll(r, sym)))
-    return t
+    """Oracle table bundle with a copy of the REFERENCE's tables (after ref_mp_start())."""
+    global _ref_tab
+    if _ref_tab is None:
+        tabs = reference("tables", (), lambda: {f: _b64(np.ctypeslib.as_array((C.c_uint8 * n).in_dll(ref(), "ref_ns_tab_" + f)))
+                                                for f, n in _TAB_SIZES})
+        arr = [_unb64(tabs[f], np.uint8) for f, _ in _TAB_SIZES]
+        _ref_tab = (tables_from_arrays(*arr), arr)
+    return _ref_tab[0]
 
 
 def tables_from_arrays(nt4, aa20, aa13, codon, codon13):
@@ -121,30 +230,89 @@ DEFAULT_NASW = dict(go=11, ge=1, io=29, fs=23, xdrop=100, end_bonus=5, sp=(8, 15
 
 
 def default_mat() -> np.ndarray:
-    """BLOSUM62 22x22 with the miniprot stop-codon row (options.c:87-88), read from the reference when present."""
-    r = ref()
-    m = np.ctypeslib.as_array((C.c_int8 * 484).in_dll(r, "ref_ns_mat_blosum62")).copy()
-    r.ref_ns_set_stop_sc(22, m.ctypes.data_as(C.c_void_p), 23)
-    return m
+    """BLOSUM62 22x22 with the miniprot stop-codon row (options.c:87-88), the reference's."""
+    def compute():
+        m = np.ctypeslib.as_array((C.c_int8 * 484).in_dll(ref(), "ref_ns_mat_blosum62")).copy()
+        ref().ref_ns_set_stop_sc(22, m.ctypes.data_as(C.c_void_p), 23)
+        return _b64(m)
+
+    return _unb64(reference("default_mat", (), compute), np.int8)
+
+
+def ref_set_stop_sc(mat: np.ndarray, sc: int) -> None:
+    """The reference's ns_set_stop_sc(22, mat, sc) (-C, options.c:87-88), in place."""
+    def compute():
+        m = mat.copy()
+        ref().ref_ns_set_stop_sc(22, m.ctypes.data_as(C.c_void_p), sc)
+        return _b64(m)
+
+    mat[:] = _unb64(reference("set_stop_sc", (mat.tobytes(), sc), compute), np.int8)
 
 
 def ref_nasw(nt: np.ndarray, aa: bytes, flag: int, mat: np.ndarray, par: dict, ss=None):
-    r = ref()
-    o = NsOpt()
-    r.ref_ns_opt_init(C.byref(o))
-    for k in ("go", "ge", "io", "fs", "xdrop", "end_bonus", "sp_null_bonus", "ie_coef"):
-        setattr(o, k, par[k])
-    for i in range(6):
-        o.sp[i] = par["sp"][i]
-    o.flag = flag
-    o.sc = mat.ctypes.data
-    rst = NsRst()
-    ssp = ss.ctypes.data_as(C.c_void_p) if ss is not None else None
-    r.ref_ns_global_gs16b(None, nt.tobytes(), len(nt), aa, len(aa), C.byref(o), ssp, C.byref(rst))
-    cig = [rst.cigar[i] for i in range(rst.n_cigar)]
-    if rst.n_cigar:
-        _libc.free(rst.cigar)
-    return rst.score, rst.nt_len, rst.aa_len, cig
+    def compute():
+        r = ref()
+        o = NsOpt()
+        r.ref_ns_opt_init(C.byref(o))
+        for k in ("go", "ge", "io", "fs", "xdrop", "end_bonus", "sp_null_bonus", "ie_coef"):
+            setattr(o, k, par[k])
+        for i in range(6):
+            o.sp[i] = par["sp"][i]
+        o.flag = flag
+        o.sc = mat.ctypes.data
+        rst = NsRst()
+        ssp = ss.ctypes.data_as(C.c_void_p) if ss is not None else None
+        r.ref_ns_global_gs16b(None, nt.tobytes(), len(nt), aa, len(aa), C.byref(o), ssp, C.byref(rst))
+        cig = [rst.cigar[i] for i in range(rst.n_cigar)]
+        if rst.n_cigar:
+            _libc.free(rst.cigar)
+        return [rst.score, rst.nt_len, rst.aa_len, cig]
+
+    parts = (np.ascontiguousarray(nt, dtype=np.uint8).tobytes(), bytes(aa), flag, mat.tobytes(), par,
+             None if ss is None else np.ascontiguousarray(ss, dtype=np.uint8).tobytes())
+    score, nt_len, aa_len, cig = reference("nasw", parts, compute)
+    return score, nt_len, aa_len, cig
+
+
+def ref_sort128x(z: np.ndarray) -> str:
+    """sha256 of what the reference's radix_sort_mp128x makes of the (n, 2) uint64 array z."""
+    def compute():
+        a = z.copy()
+        ref().ref_radix_sort_mp128x(a.ctypes.data_as(C.c_void_p), C.c_void_p(a.ctypes.data + 16 * len(a)))
+        return digest(a.tobytes())
+
+    return reference("sort128x", (z.tobytes(),), compute)
+
+
+class _Mp64(C.Structure):  # mp64_v
+    _fields_ = [("n", C.c_int32), ("m", C.c_int32), ("a", C.POINTER(C.c_uint64))]
+
+
+def _take_mp64(v: _Mp64):
+    a = np.ctypeslib.as_array(v.a, shape=(v.n,)).copy() if v.n else np.zeros(0, np.uint64)
+    if v.a:
+        _libc.free(v.a)
+    return [v.n, digest(a.tobytes())]
+
+
+def ref_sketch_prot(seq: bytes, k: int, m: int):
+    """(n, sha256 of the n uint64s) of the reference's mp_sketch_prot."""
+    def compute():
+        v = _Mp64()
+        ref().ref_mp_sketch_prot(None, seq, len(seq), k, m, C.byref(v))
+        return _take_mp64(v)
+
+    return tuple(reference("sketch_prot", (seq, k, m), compute))
+
+
+def ref_sketch_nt4(nt: np.ndarray, k: int, m: int, bbit: int, boff: int):
+    """(n, sha256 of the n uint64s) of the reference's mp_sketch_nt4 (min_aa_len 30)."""
+    def compute():
+        v = _Mp64()
+        ref().ref_mp_sketch_nt4(None, nt.ctypes.data_as(C.c_void_p), C.c_int64(len(nt)), 30, k, m, bbit, C.c_int64(boff), C.byref(v))
+        return _take_mp64(v)
+
+    return tuple(reference("sketch_nt4", (nt.tobytes(), k, m, bbit, boff), compute))
 
 
 def ora_nasw(tab: OraTab, nt: np.ndarray, aa: bytes, flag: int, mat: np.ndarray, par: dict, ss=None):
@@ -257,15 +425,19 @@ def chain_par(mode: str, **over) -> ChainPar:
 
 
 def ref_chain(par: ChainPar, a: np.ndarray):
-    r = ref()
-    n = len(a)
-    buf = r.ref_kmalloc(None, max(8 * n, 8))  # mp_chain frees its input
-    C.memmove(buf, a.ctypes.data, 8 * n)
-    n_u = C.c_int32(0)
-    u = C.c_void_p(0)
-    b = r.ref_mp_chain(par.max_dist_x, par.max_dist_y, par.bw, par.max_skip, par.max_iter, par.min_cnt, par.min_sc,
-                       par.chn_coef_log, par.is_spliced, par.kmer, par.bbit, n, buf, C.byref(n_u), C.byref(u), None)
-    return _take_chain(n_u.value, u.value, b)
+    def compute():
+        r = ref()
+        n = len(a)
+        buf = r.ref_kmalloc(None, max(8 * n, 8))  # mp_chain frees its input
+        C.memmove(buf, a.ctypes.data, 8 * n)
+        n_u = C.c_int32(0)
+        u = C.c_void_p(0)
+        b = r.ref_mp_chain(par.max_dist_x, par.max_dist_y, par.bw, par.max_skip, par.max_iter, par.min_cnt, par.min_sc,
+                           par.chn_coef_log, par.is_spliced, par.kmer, par.bbit, n, buf, C.byref(n_u), C.byref(u), None)
+        return [_b64(x) for x in _take_chain(n_u.value, u.value, b)]
+
+    u, b = reference("chain", (par, a.tobytes()), compute)
+    return _unb64(u, np.uint64), _unb64(b, np.uint64)
 
 
 def _take_chain(n_u, u_ptr, b_ptr):

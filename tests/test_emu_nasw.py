@@ -7,8 +7,6 @@ import pytest
 import build_hostcheck
 import oracle_lib as ol
 
-pytestmark = pytest.mark.skipif(not ol.have_ref(), reason="needs oracle/_ref for the tables")
-
 
 @pytest.fixture(scope="module")
 def hc():
@@ -20,12 +18,11 @@ def hc():
 
 
 def emu(hc, nt, aa, flag, Ccols, mat, par):
-    r = ol.ref()
+    tab = ol.ref_tables()
     sp = (C.c_int32 * 6)(*par["sp"])
     sc, ntl, aal = C.c_int(), C.c_int(), C.c_int()
     cig = (C.c_uint32 * (len(nt) + len(aa) + 16))()
-    n = hc.emu_nasw(C.addressof(C.c_uint8.in_dll(r, "ref_ns_tab_nt4")), C.addressof(C.c_uint8.in_dll(r, "ref_ns_tab_aa20")),
-                    C.addressof(C.c_uint8.in_dll(r, "ref_ns_tab_codon")), mat.ctypes.data, C.addressof(sp), par["go"], par["ge"],
+    n = hc.emu_nasw(tab.nt4, tab.aa20, tab.codon, mat.ctypes.data, C.addressof(sp), par["go"], par["ge"],
                     par["io"], par["fs"], par["xdrop"], par["end_bonus"], par["ie_coef"], flag, Ccols,
                     nt.ctypes.data, len(nt), aa, len(aa), C.addressof(sc), C.addressof(ntl), C.addressof(aal), C.addressof(cig), len(cig))
     return sc.value, ntl.value, aal.value, [cig[i] for i in range(n)]
@@ -121,15 +118,14 @@ def random_spsc(rng, nt, max_sc=14, p_set=0.3):
 
 
 def emu_ss(hc, nt, aa, flag, Ccols, mat, par, ss):
-    r = ol.ref()
+    tab = ol.ref_tables()
     hc.emu_nasw_ss.restype = C.c_int
     hc.emu_nasw_ss.argtypes = [C.c_void_p] * 5 + [C.c_int] * 6 + [C.c_float, C.c_int, C.c_int, C.c_void_p, C.c_int, C.c_char_p, C.c_int] + \
         [C.c_void_p] * 4 + [C.c_int, C.c_void_p, C.c_int]
     sp = (C.c_int32 * 6)(*par["sp"])
     sc, ntl, aal = C.c_int(), C.c_int(), C.c_int()
     cig = (C.c_uint32 * (len(nt) + len(aa) + 16))()
-    n = hc.emu_nasw_ss(C.addressof(C.c_uint8.in_dll(r, "ref_ns_tab_nt4")), C.addressof(C.c_uint8.in_dll(r, "ref_ns_tab_aa20")),
-                       C.addressof(C.c_uint8.in_dll(r, "ref_ns_tab_codon")), mat.ctypes.data, C.addressof(sp), par["go"], par["ge"],
+    n = hc.emu_nasw_ss(tab.nt4, tab.aa20, tab.codon, mat.ctypes.data, C.addressof(sp), par["go"], par["ge"],
                        par["io"], par["fs"], par["xdrop"], par["end_bonus"], par["ie_coef"], flag, Ccols,
                        nt.ctypes.data, len(nt), aa, len(aa), C.addressof(sc), C.addressof(ntl), C.addressof(aal), C.addressof(cig), len(cig),
                        ss.ctypes.data, par["sp_null_bonus"])

@@ -1,5 +1,5 @@
 """GPU parity on the shapes of BASELINE.json's configurations (SURVEY 8d): the whole path (FASTA proteins -> PAF through
-mpb_map_file) against the reference CLI run on the same box, byte for byte.
+mpb_map_file) against the reference CLI (run on the same box, or its recorded output digest), byte for byte.
 
   C5   100 Mbp, 1000 proteins at 60 % identity with 2 % frameshifts (full size): every scoring branch / CIGAR operation
   C4s  the long-intron stress shape (one 50-150 kbp intron per gene, 400 kbp slots) under the -G x -e sweep
@@ -16,7 +16,7 @@ sys.path.insert(0, os.path.join(ROOT, "tools"))
 
 import oracle_lib as ol  # noqa: E402
 
-pytestmark = [pytest.mark.gpu, pytest.mark.skipif(not os.path.exists(ol.REF_BIN), reason="reference binary not present")]
+pytestmark = pytest.mark.gpu
 
 
 @pytest.fixture(scope="module")

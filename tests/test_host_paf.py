@@ -11,7 +11,6 @@ from miniprot_b200 import synth
 
 HERE = os.path.dirname(os.path.abspath(__file__))
 GOLD = os.path.join(HERE, "golden")
-DATA = os.path.join(ol.ORA_DIR, "_ref", "data")
 
 
 @pytest.fixture(scope="module")
@@ -26,10 +25,9 @@ def run(hc, g, p, out, flag=0, max_intron=0, auto=0, sp=-1, mini_batch=0):
     return open(out, "rb").read()
 
 
-@pytest.mark.skipif(not os.path.exists(os.path.join(DATA, "DPP3-hs.gen.fa.gz")), reason="bundled DPP3 pair not present (oracle/_ref/data)")
 @pytest.mark.parametrize("name,kw", [("DPP3_default", {}), ("DPP3_j2", dict(sp=2)), ("DPP3_G2k", dict(max_intron=2000))])
 def test_dpp3_golden(hc, tmp_path, name, kw):
-    got = run(hc, os.path.join(DATA, "DPP3-hs.gen.fa.gz"), os.path.join(DATA, "DPP3-mm.pep.fa.gz"), str(tmp_path / "o.paf"), **kw)
+    got = run(hc, ol.DPP3_GEN, ol.DPP3_PEP, str(tmp_path / "o.paf"), **kw)
     assert got == open(os.path.join(GOLD, name + ".paf"), "rb").read()
 
 
@@ -65,9 +63,8 @@ def test_other_output_formats_golden(hc, tmp_path, fmt, monkeypatch):
     want = gzip.open(gold + ".gz", "rb").read() if os.path.exists(gold + ".gz") else open(gold, "rb").read()
     assert run(hc, g, p, str(tmp_path / "o.txt"), flag=flag) == want
     assert run(hc, g, p, str(tmp_path / "o2.txt"), flag=flag, mini_batch=1200) == want  # the hit counter runs across mini-batches
-    if os.path.exists(os.path.join(DATA, "DPP3-hs.gen.fa.gz")):
-        got = run(hc, os.path.join(DATA, "DPP3-hs.gen.fa.gz"), os.path.join(DATA, "DPP3-mm.pep.fa.gz"), str(tmp_path / "d.txt"), flag=flag)
-        assert got == open(os.path.join(GOLD, f"DPP3_{fmt}.txt"), "rb").read()
+    got = run(hc, ol.DPP3_GEN, ol.DPP3_PEP, str(tmp_path / "d.txt"), flag=flag)
+    assert got == open(os.path.join(GOLD, f"DPP3_{fmt}.txt"), "rb").read()
 
 
 @pytest.mark.parametrize("extra", [0, 1, 2, 3, 4])

@@ -1,5 +1,6 @@
 """CPU: the product library loads, exports every symbol of include/*.h, and its tables / defaults equal the reference's."""
 import ctypes as C
+import json
 import os
 import re
 
@@ -32,42 +33,54 @@ def test_exports_every_declared_symbol(L):
         C.c_uint8.in_dll(L, g)
 
 
-@pytest.mark.skipif(not ol.have_ref(), reason="needs oracle/_ref")
-def test_tables_and_defaults_equal_reference(L):
-    r = ol.ref()
+TABLES = (("ns_tab_nt4", 256), ("ns_tab_aa20", 256), ("ns_tab_aa13", 256), ("ns_tab_codon", 64), ("ns_tab_codon13", 64), ("ns_tab_a2r", 22))
+GSIZES = (1000, 10**8, 3 * 10**9, 10**11)
+
+
+def _opt_fields(o):
+    return {f: (bytes(v).hex() if f == "mat" else v.decode() if isinstance(v, bytes) else v) for f, _ in o._fields_ for v in [getattr(o, f)]}
+
+
+def _defaults(L, pre=""):
+    """Translation tables of several genetic codes, option defaults and -I's max intron, through library L (symbols prefixed `pre`)."""
+    fn = lambda name: getattr(L, pre + name)  # noqa: E731
+    d = {"tables": {}}
     for code in (1, 2, 4, 11, 33):
-        assert L.ns_make_tables(code) == 0 and r.ref_ns_make_tables(code) == 0
-        for name, n in (("ns_tab_nt4", 256), ("ns_tab_aa20", 256), ("ns_tab_aa13", 256), ("ns_tab_codon", 64), ("ns_tab_codon13", 64), ("ns_tab_a2r", 22)):
-            a = bytes((C.c_uint8 * n).in_dll(L, name))
-            b = bytes((C.c_uint8 * n).in_dll(r, "ref_" + name))
-            assert a == b, (code, name)
-    assert L.ns_make_tables(7) == r.ref_ns_make_tables(7) == -2
-    L.ns_make_tables(1), r.ref_ns_make_tables(1)
-    assert bytes((C.c_int8 * 484).in_dll(L, "ns_mat_blosum62")) == bytes((C.c_int8 * 484).in_dll(r, "ref_ns_mat_blosum62"))
-    mo, ro = mp.MapOpt(), mp.MapOpt()
-    L.mp_mapopt_init(C.byref(mo)), r.ref_mp_mapopt_init(C.byref(ro))
-    for f, _ in mp.MapOpt._fields_:
-        a, b = getattr(mo, f), getattr(ro, f)
-        if f == "mat":
-            assert bytes(a) == bytes(b)
-        else:
-            assert a == b, f
-    io, rio = mp.IdxOpt(), mp.IdxOpt()
-    L.mp_idxopt_init(C.byref(io)), r.ref_mp_idxopt_init(C.byref(rio))
-    assert bytes(io) == bytes(rio)
-    no, rno = mp.NsOpt(), mp.NsOpt()
-    L.ns_opt_init(C.byref(no)), r.ref_ns_opt_init(C.byref(rno))
-    for f in ("go", "ge", "io", "fs", "xdrop", "end_bonus", "asize", "sp_null_bonus", "ie_coef"):
-        assert getattr(no, f) == getattr(rno, f), f
-    assert list(no.sp) == list(rno.sp)
-    r.ref_mp_mapopt_set_max_intron.argtypes = [C.c_void_p, C.c_int64]
-    C.c_int32.in_dll(r, "ref_mp_verbose").value = 1
-    for gsize in (1000, 10**8, 3 * 10**9, 10**11):
-        L.mp_mapopt_set_max_intron(C.byref(mo), gsize), r.ref_mp_mapopt_set_max_intron(C.addressof(ro), gsize)
-        assert (mo.max_intron, mo.bw) == (ro.max_intron, ro.bw)
+        assert fn("ns_make_tables")(code) == 0
+        d["tables"][str(code)] = {name: bytes((C.c_uint8 * n).in_dll(L, pre + name)).hex() for name, n in TABLES}
+    d["make_tables_7"] = fn("ns_make_tables")(7)
+    fn("ns_make_tables")(1)
+    d["blosum62"] = bytes((C.c_int8 * 484).in_dll(L, pre + "ns_mat_blosum62")).hex()
+    mo, io, no = mp.MapOpt(), mp.IdxOpt(), mp.NsOpt()
+    fn("mp_mapopt_init")(C.byref(mo))
+    fn("mp_idxopt_init")(C.byref(io))
+    fn("ns_opt_init")(C.byref(no))
+    d["mapopt"], d["idxopt"] = _opt_fields(mo), bytes(io).hex()
+    d["nsopt"] = {f: getattr(no, f) for f in ("go", "ge", "io", "fs", "xdrop", "end_bonus", "asize", "sp_null_bonus", "ie_coef")}
+    d["nsopt"]["sp"] = list(no.sp)
+    if pre:
+        fn("mp_mapopt_set_max_intron").argtypes = [C.c_void_p, C.c_int64]
+    C.c_int32.in_dll(L, pre + "mp_verbose").value = 1
+    d["max_intron_bw"] = []
+    for gsize in GSIZES:
+        fn("mp_mapopt_set_max_intron")(C.addressof(mo) if pre else C.byref(mo), gsize)
+        d["max_intron_bw"].append([mo.max_intron, mo.bw])
+    return d
 
 
-@pytest.mark.skipif(not ol.have_ref(), reason="needs oracle/_ref")
+def test_tables_and_defaults_equal_reference(L):
+    ours = json.loads(json.dumps(_defaults(L)))
+    want = ol.reference("defaults", (), lambda: _defaults(ol.ref(), "ref_"))
+    for code in want["tables"]:
+        for name, _ in TABLES:
+            assert ours["tables"][code][name] == want["tables"][code][name], (code, name)
+    assert ours["make_tables_7"] == want["make_tables_7"] == -2
+    for k in ("blosum62", "idxopt", "nsopt", "max_intron_bw"):
+        assert ours[k] == want[k], k
+    for f in want["mapopt"]:
+        assert ours["mapopt"][f] == want["mapopt"][f], f
+
+
 def test_index_file_is_byte_identical(L, tmp_path):
     """mp_idx_build + mp_idx_dump vs the reference's -d output on a small synthetic genome (ki/kb order is part of the contract)."""
     import subprocess
@@ -78,9 +91,13 @@ def test_index_file_is_byte_identical(L, tmp_path):
     mi = mp.idx_load(g, 4)
     assert L.mp_idx_dump(ours.encode(), mi) == 0
     L.mp_idx_destroy(mi)
-    subprocess.run([ol.REF_BIN, "-t4", "-d", ref, g], check=True, stderr=subprocess.DEVNULL)
-    assert open(ours, "rb").read() == open(ref, "rb").read()
-    mi2 = L.mp_idx_restore(ref.encode())
+
+    def ref_dump():
+        subprocess.run([ol.REF_BIN, "-t4", "-d", ref, g], check=True, stderr=subprocess.DEVNULL)
+        return ol.file_digest(ref)
+
+    assert ol.file_digest(ours) == ol.reference("idx_dump", (ol.file_digest(g),), ref_dump)
+    mi2 = L.mp_idx_restore((ref if os.path.exists(ref) else ours).encode())
     assert mi2 and mi2.contents.n_kb > 0
     L.mp_idx_destroy(mi2)
 
@@ -94,34 +111,39 @@ def test_no_gpu_means_loud_failure(L):
         mp.Context(0)
 
 
-@pytest.mark.skipif(not ol.have_ref(), reason="needs oracle/_ref")
+class Spsc(C.Structure):
+    _fields_ = [("n", C.c_uint32), ("m", C.c_uint32), ("a", C.POINTER(C.c_uint64))]
+
+
+def _spsc(L, pre, g, sp):
+    """(io, io_end) after mp_set_spsc and the per-strand arrays (length, sha256) it leaves in the index, for keep_io 0 and 1."""
+    fn = getattr(L, pre + "mp_idx_load")
+    fn.restype = C.POINTER(mp.Idx)
+    mi = fn(g.encode(), C.byref(mp.idxopt()), 4)
+    out = []
+    for keep_io in (0, 1):
+        mo = mp.mapopt()
+        getattr(L, pre + "mp_set_spsc")(sp.encode(), mi, C.byref(mo), keep_io)
+        sa = C.cast(mi.contents.nt.contents.spsc, C.POINTER(Spsc))
+        arrays = [[sa[j].n, ol.digest(C.string_at(sa[j].a, 8 * sa[j].n) if sa[j].n else b"")] for j in range(2 * mi.contents.nt.contents.n_ctg)]
+        out.append([[mo.io, mo.io_end], arrays])
+    getattr(L, pre + "mp_idx_destroy")(mi)
+    return out
+
+
 def test_splice_score_reader_equals_reference(L, tmp_path):
     """mp_set_spsc / mp_ntseq_read_spsc (index.c:239-248, ntseq.c:234-296): option side effects and the sorted per-strand arrays."""
     from miniprot_b200 import synth
-    r = ol.ref()
     g, _ = synth.generate(synth.CONFIGS["tiny"], str(tmp_path))
     sp = synth.make_spsc(g, str(tmp_path / "t.spsc"), seed=3, p_site=0.2, p_noise=0.001)
-
-    class Spsc(C.Structure):
-        _fields_ = [("n", C.c_uint32), ("m", C.c_uint32), ("a", C.POINTER(C.c_uint64))]
-
-    io = mp.idxopt()
-    for fn in (L.mp_idx_load, r.ref_mp_idx_load):
-        fn.restype = C.POINTER(mp.Idx)
-    a, b = L.mp_idx_load(g.encode(), C.byref(io), 4), r.ref_mp_idx_load(g.encode(), C.byref(io), 4)
-    for keep_io in (0, 1):
-        mo, ro = mp.mapopt(), mp.mapopt()
-        L.mp_set_spsc(sp.encode(), a, C.byref(mo), keep_io), r.ref_mp_set_spsc(sp.encode(), b, C.byref(ro), keep_io)
-        assert (mo.io, mo.io_end) == (ro.io, ro.io_end) == ((29, 19) if keep_io else (39, 29))
-        n_ctg = a.contents.nt.contents.n_ctg
-        sa, sb = C.cast(a.contents.nt.contents.spsc, C.POINTER(Spsc)), C.cast(b.contents.nt.contents.spsc, C.POINTER(Spsc))
-        tot = 0
-        for j in range(2 * n_ctg):
-            assert sa[j].n == sb[j].n, j
-            assert [sa[j].a[k] for k in range(sa[j].n)] == [sb[j].a[k] for k in range(sb[j].n)], j
-            tot += sa[j].n
-        assert tot > 1000
-    L.mp_idx_destroy(a)
+    ours = json.loads(json.dumps(_spsc(L, "", g, sp)))
+    want = ol.reference("spsc", (ol.file_digest(g), ol.file_digest(sp)), lambda: _spsc(ol.ref(), "ref_", g, sp))
+    for keep_io, ((io, arrays), (wio, warrays)) in enumerate(zip(ours, want)):
+        assert io == wio == ([29, 19] if keep_io else [39, 29])
+        assert len(arrays) == len(warrays)
+        for j, (a, w) in enumerate(zip(arrays, warrays)):
+            assert a == w, j
+        assert sum(n for n, _ in warrays) > 1000
 
 
 def test_build_record_matches_the_loaded_library():

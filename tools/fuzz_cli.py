@@ -2,7 +2,8 @@
 UNMODIFIED main.c linked against tests/_build/libhostcheck.so (the product's host sources -- options, index builder, .mpi I/O, hit
 bookkeeping, alignment planner, statistics, all output formats -- with the C oracle as stage backend) against the reference binary
 oracle/_ref/miniprot, same random options, same random synthetic inputs; stdout must be byte-identical.
-Needs /root/reference (to compile main.c) and oracle/_ref.  Test infrastructure, not part of the product.
+Needs oracle/_ref (the reference binary and the CLI, built by oracle/Makefile where the reference sources are present).  Test
+infrastructure, not part of the product.
 
 usage: python tools/fuzz_cli.py [seed] [n_iterations] [workdir]"""
 import os
@@ -18,19 +19,18 @@ sys.path.insert(0, os.path.join(ROOT, "tests"))
 import build_hostcheck  # noqa: E402
 from miniprot_b200 import synth  # noqa: E402
 
-REF_SRC = os.environ.get("MPB_REFERENCE", "/root/reference")
 REF_BIN = os.path.join(ROOT, "oracle", "_ref", "miniprot")
 CLI = os.path.join(ROOT, "oracle", "_ref", "miniprot_hostcheck_cli")  # compiled reference source: output under oracle/_ref like the other reference builds
 
 
 def build_cli():
     """oracle/_ref/miniprot_hostcheck_cli = reference main.c (compiled where it lies) + tests/_build/libhostcheck.so; the recipe is
-    oracle/Makefile (target hostcheck_cli)"""
+    oracle/Makefile (target hostcheck_cli, made by __graft_entry__.build() where the reference sources are present; with
+    MPB_REFERENCE=<reference source directory> it is remade here).  None if it has not been built."""
     build_hostcheck.build()
-    if not os.path.exists(os.path.join(REF_SRC, "main.c")):
-        return None
-    subprocess.run(["make", "-s", "-C", os.path.join(ROOT, "oracle"), "hostcheck_cli", "REF=" + REF_SRC], check=True)
-    return CLI
+    if os.environ.get("MPB_REFERENCE"):
+        subprocess.run(["make", "-s", "-C", os.path.join(ROOT, "oracle"), "hostcheck_cli", "REF=" + os.environ["MPB_REFERENCE"]], check=True)
+    return CLI if os.path.exists(CLI) else None
 
 
 def random_inputs(rng, d):
@@ -160,7 +160,7 @@ def random_options(rng, g, d):
 def fuzz(seed, n_it, workdir=None):
     cli = os.environ.get("MPB_FUZZ_CLI") or build_cli()  # MPB_FUZZ_CLI: e.g. the same program built with -fsanitize=address,undefined
     if cli is None or not os.path.exists(REF_BIN):
-        print("needs the reference sources (main.c) and oracle/_ref/miniprot")
+        print("needs oracle/_ref/miniprot and oracle/_ref/miniprot_hostcheck_cli (oracle/Makefile)")
         return 0, 0
     rng = np.random.default_rng(seed)
     bad = n_ref_abort = 0

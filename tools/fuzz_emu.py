@@ -51,7 +51,7 @@ def fuzz(seed, n_it):
         par = random_par(rng)
         mat = ol.default_mat()
         if rng.random() < 0.3:  # -C: stop-codon score scale (options.c:87-88)
-            ol.ref().ref_ns_set_stop_sc(22, mat.ctypes.data_as(C.c_void_p), int(rng.integers(1, 60)))
+            ol.ref_set_stop_sc(mat, int(rng.integers(1, 60)))
         shape = rng.random()
         if LONG:  # MPB_FUZZ_PROFILE=long: several column passes, thousands of rows, long introns, slices cut anywhere
             al_max = 300 if shape < 0.4 else 700 if shape < 0.8 else 1500

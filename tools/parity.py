@@ -4,23 +4,23 @@ same synthetic inputs, byte for byte.  Test / measurement infrastructure: the re
   python tools/parity.py CONFIG [--opt "-I"] [--opt "-G 50k -e 2k"] ... [--dir DIR] [--json OUT]
 
 Every --opt string is one run of both sides with those reference CLI options (a subset is understood on our side:
--I, -G, -e, -j, -S).  Prints one line per run with the md5s and the wall times; exit status 1 on any mismatch."""
+-I, -G, -e, -j, -S).  Prints one line per run with the md5s and the wall times; exit status 1 on any mismatch.  Where the
+reference is not built, its output digests recorded in tests/golden stand in for it (tests/oracle_lib.py ref_cli; no times then)."""
 from __future__ import annotations
 
 import argparse
 import hashlib
 import json
 import os
-import subprocess
 import sys
 import time
 
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 sys.path.insert(0, ROOT)
+sys.path.insert(0, os.path.join(ROOT, "tests"))
 import miniprot_b200 as mp  # noqa: E402
+import oracle_lib as ol  # noqa: E402
 from miniprot_b200 import synth  # noqa: E402
-
-REF_BIN = os.path.join(ROOT, "oracle", "_ref", "miniprot")
 
 
 def parse_num(s: str) -> int:
@@ -91,29 +91,28 @@ def run_config(cfg: str, opts, d: str, threads: int, ctx=None, keep=False):
         mp.map_file(ctx, mi, p, out, mo)
         t_ours = time.time() - t0
         st = ctx.stats()
-        t0 = time.time()
-        ref = subprocess.run([REF_BIN, f"-t{threads}", *o.split(), mpi, p], check=True, capture_output=True)
-        t_ref = time.time() - t0
+        want = ol.ref_cli(o.split(), g, p, threads=threads, index=mpi)  # the reference restores the same index file
+        t_ref = want.get("s")
         t_ref_map = None
-        for line in ref.stderr.decode().splitlines():  # "[M::mp_idx_restore@0.210*1.00] ..." (index.c:227): mapping = wall - restore
+        for line in want.get("err", b"").decode().splitlines():  # "[M::mp_idx_restore@0.210*1.00] ..." (index.c:227): mapping = wall - restore
             if "mp_idx_restore@" in line:
                 try:
                     t_ref_map = t_ref - float(line.split("mp_idx_restore@")[1].split("*")[0])
                 except Exception:
                     pass
         ours = open(out, "rb").read()
-        same = ours == ref.stdout
-        row = {"config": cfg, "opt": o, "identical": same, "n_proteins": n_prot, "paf_lines": ours.count(b"\n"), "ref_lines": ref.stdout.count(b"\n"),
-               "md5_ours": hashlib.md5(ours).hexdigest(), "md5_ref": hashlib.md5(ref.stdout).hexdigest(), "ours_s": round(t_ours, 3), "ref_s": round(t_ref, 3),
-               "ref_map_s": None if t_ref_map is None else round(t_ref_map, 3), "ref_threads": threads,
+        same = hashlib.md5(ours).hexdigest() == want["md5"]
+        row = {"config": cfg, "opt": o, "identical": same, "n_proteins": n_prot, "paf_lines": ours.count(b"\n"), "ref_lines": want["lines"],
+               "md5_ours": hashlib.md5(ours).hexdigest(), "md5_ref": want["md5"], "ours_s": round(t_ours, 3), "ref_s": None if t_ref is None else round(t_ref, 3),
+               "ref_map_s": None if t_ref_map is None else round(t_ref_map, 3), "ref_threads": threads if t_ref is not None else None,
                "anchors_per_protein": st.n_anchors / max(n_prot, 1), "dp_gcells": (st.dp_cells_ext + st.dp_cells_tb) / 1e9,
                "wall_ms": [round(x, 1) for x in st.ms_wall], "gen_s": round(t_gen, 1), "idx_build_s": round(t_build, 1), "idx_load_s": round(t_load, 2),
                "idx_upload_s": round(t_up, 2)}
-        if not same:
-            a, b = ours.decode().splitlines(), ref.stdout.decode().splitlines()
+        if not same and "out" in want:
+            a, b = ours.decode().splitlines(), want["out"].decode().splitlines()
             row["first_diffs"] = [(x[:160], y[:160]) for x, y in zip(a, b) if x != y][:3]
             if keep:
-                open(os.path.join(d, "ref.paf"), "wb").write(ref.stdout)
+                open(os.path.join(d, "ref.paf"), "wb").write(want["out"])
         rows.append(row)
         print(json.dumps(row), flush=True)
     mp.lib().mp_idx_destroy(mi)
